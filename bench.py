@@ -3,6 +3,7 @@
 --gpus 8; [3] with --bands 12) and MPix/s of 16x16-chunk grid inference (configs[4], --mode infer).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--mode train|infer] [--bands 3|12] [--impl engine|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 train: a "step" = SSRESRGANModel.feed_data kernels (uint8 -> float/255, USM sharpen) + optimize_parameters
@@ -278,8 +279,7 @@ def cpu_baseline(mode, bands, steps, warm):
 def run_reference(args, rank, world):
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 3))
-    warm = 1 if args.warmup > 0 else 0
+    steps, warm = args.steps, args.warmup
     cb = cpu_baseline(args.mode, args.bands, steps, warm)
     t = cb.pop("t")
     cb.pop("steps")
@@ -322,6 +322,38 @@ class Harness:
         return ms.item()
 
 
+def dump_outputs(path, arrays):
+    """--dump-outputs: each array as <path>/<name>.npy in float32 (float64 for loss scalars), so two builds can be compared"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        np.save(os.path.join(path, f"{name}.npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+
+
+def train_state(tr):
+    """every tensor a training step reads and updates: parameters, spectral-norm vectors, EMA copy, Adam moments (the packed
+    weights are rebuilt from these at the start of each step)"""
+    return tr.replicated_tensors() + [t for o in (tr.opt_g, tr.opt_d) for t in (o.m.flat, o.v.flat)]
+
+
+def restore_train_state(tr, saved):
+    for t, s in zip(train_state(tr), saved):
+        t.copy_(s)
+    for o in (tr.opt_g, tr.opt_d):
+        o.step_count = 0
+        o.sync_device_hyper()
+
+
+def train_outputs(model):
+    """what a caller of optimize_parameters receives after the step: the generator output and the loss scalars.  The updated
+    weights are optimizer state, not an output, and are left out: one Adam step from zero moments moves every weight by
+    lr * sign(gradient), so a gradient element at the rounding level of the atomic reductions flips by 2 * lr."""
+    out = {"output": model.output.float()}
+    out.update({k: torch.tensor(v, dtype=torch.float64) for k, v in model.get_current_log().items()})
+    return out
+
+
 def roofline_entry(kernel, flop, ms, count, peak, peak_src, extra=None):
     ach = flop / (ms / 1e3) / 1e12 if ms > 0 else None
     d = {"kernel": kernel, "bound": "tensor", "achieved": ach, "peak": peak, "unit": "TFLOP/s", "frac": ach / peak if ach else None,
@@ -332,13 +364,14 @@ def roofline_entry(kernel, flop, ms, count, peak, peak_src, extra=None):
     return d
 
 
-def measure_train(args, bands, rank, world, local, lib, L, harness, steps, warmup):
+def measure_train(args, bands, rank, world, local, lib, L, harness, steps, warmup, dump=None):
     from satlas_super_resolution_b200.ops import cur_stream
     from satlas_super_resolution_b200.registry import build_model
     B = args.batch
     torch.manual_seed(rank)            # ssr/utils/options.py:81 seeds every rank with manual_seed + rank; rank 0's init is broadcast
     model = build_model(model_opt(bands, not args.no_graph, world > 1))
     tr = model.trainer
+    initial = [t.clone() for t in train_state(tr)]
     lr_h, hr_h = synthetic_batch(B, rank, bands)
     data = {"lr": lr_h.pin_memory(), "hr": hr_h.pin_memory()}
     it = [0]
@@ -360,8 +393,19 @@ def measure_train(args, bands, rank, world, local, lib, L, harness, steps, warmu
         step_resident()
         torch.cuda.synchronize()
         log(f"warm-up step {i} done")
-    ms_total = harness.timed(step_resident, steps)
+    # The last timed step starts again from the seeded initial state (restored between two timed spans): the weight and
+    # spectral-norm reductions sum with f32 atomics in no fixed order, and the GAN game amplifies those last-bit differences
+    # step by step, so only a step from a fixed state computes the same outputs in every run.  A step's work does not depend
+    # on the weight values.
+    ms_total = harness.timed(step_resident, steps - 1) if steps > 1 else 0.0
+    restore_train_state(tr, initial)
+    del initial
+    ms_total += harness.timed(step_resident, 1)
     log(f"resident timing done: {ms_total / steps:.2f} ms/step")
+    if dump:
+        outs = train_outputs(model)           # every rank: the loss read-back reduces over ranks
+        if rank == 0:
+            dump_outputs(dump, outs)
     # The end-to-end loop has the host on the critical path every step (H2D, graph launch, loss read-back): ONE stall of the host thread
     # (another process holding a driver lock for tens of ms) shifts a 20-step average by several per cent -- one run of the pool showed
     # 24 instead of 16.7 ms.  Two K-step passes; the faster one is reported, both are listed in the line (e2e.passes_ms_per_step).
@@ -464,7 +508,7 @@ def train_rooflines(m, bands, peak, peak_src):
     return main, others
 
 
-def measure_infer(args, rank, world, harness, steps, warmup):
+def measure_infer(args, rank, world, harness, steps, warmup, dump=None):
     from satlas_super_resolution_b200 import weights
     from satlas_super_resolution_b200.archs import SSR_RRDBNet
     from satlas_super_resolution_b200.infer import infer_grid
@@ -475,9 +519,10 @@ def measure_infer(args, rank, world, harness, steps, warmup):
     lr_h = synthetic_batch(256, 1000 + rank)[0].pin_memory()
     lr_d = lr_h.cuda()
     host_canvas = torch.empty((2048, 2048, 3), dtype=torch.uint8).pin_memory()
+    last = [None]
 
     def step_resident():
-        infer_grid(net, lr_d, batch=args.infer_batch)
+        last[0] = infer_grid(net, lr_d, batch=args.infer_batch)
 
     def step_e2e():
         host_canvas.copy_(infer_grid(net, lr_h, batch=args.infer_batch), non_blocking=True)
@@ -485,6 +530,9 @@ def measure_infer(args, rank, world, harness, steps, warmup):
     for _ in range(warmup):
         step_resident()
     ms = harness.timed(step_resident, steps) / steps
+    if dump and rank == 0:
+        dump_outputs(dump, {"canvas": last[0]})      # the stitched uint8 [2048, 2048, 3] tile, 48 MiB as float32
+    last[0] = None
     for _ in range(2):
         step_e2e()
     ms_e2e = harness.timed(step_e2e, steps) / steps
@@ -525,7 +573,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="train mode: skip the attached inference / 12-band measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the headline measurement computed in its last timed step to "
+                                                          "DIR/<name>.npy (rank 0), for comparing two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl engine")
     rank, world, local = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":
         run_reference(args, rank, world)
@@ -547,7 +601,7 @@ def main():
         sampler.start()
 
     if args.mode == "infer":
-        m = measure_infer(args, rank, world, harness, args.steps, args.warmup)
+        m = measure_infer(args, rank, world, harness, args.steps, args.warmup, args.dump_outputs)
         sampler.stop_flag = True
         if rank == 0:
             blk = infer_block(m, world, peak_sus, peak_note, args.steps, args.warmup)
@@ -568,26 +622,26 @@ def main():
         return
 
     bands = args.bands
-    m = measure_train(args, bands, rank, world, local, lib, L, harness, args.steps, args.warmup)
+    m = measure_train(args, bands, rank, world, local, lib, L, harness, args.steps, args.warmup, args.dump_outputs)
     sampler.stop_flag = True
     clocks = sampler.summary() if rank == 0 else None
     extras = {}
     if not args.no_extras:
-        # the other two halves of BASELINE.json's metric, measured in the same run (shorter: they are attachments, not the headline)
-        k = max(3, min(args.steps, 10))
+        # the other two halves of BASELINE.json's metric, measured in the same run
+        k, w = args.steps, args.warmup
         del m["model"]
         torch.cuda.empty_cache()
-        mi = measure_infer(args, rank, world, harness, k, 3)
+        mi = measure_infer(args, rank, world, harness, k, w)
         if rank == 0:
-            extras["infer"] = infer_block(mi, world, peak_sus, peak_note, k, 3)
+            extras["infer"] = infer_block(mi, world, peak_sus, peak_note, k, w)
         other = 12 if bands == 3 else 3
-        mo = measure_train(args, other, rank, world, local, lib, L, harness, k, 3)
+        mo = measure_train(args, other, rank, world, local, lib, L, harness, k, w)
         if rank == 0:
             fo = flops(other)
             main_o, _ = train_rooflines(mo, other, peak_sus, peak_note)
             extras["train_12band" if other == 12 else "train_rgb"] = {
                 "metric": "img-pairs/sec 8-frame ESRGAN 4x train", "value": mo["B"] * world / (mo["ms_step"] / 1e3), "unit": "img-pairs/s",
-                "ms_per_step": mo["ms_step"], "steps": k, "warmup": 3, "config": dict(train_config(other), batch_per_gpu=mo["B"]),
+                "ms_per_step": mo["ms_step"], "steps": k, "warmup": w, "config": dict(train_config(other), batch_per_gpu=mo["B"]),
                 "e2e": {"value": mo["B"] * world / (mo["ms_e2e"] / 1e3), "unit": "img-pairs/s", "h2d_bytes_per_step": mo["h2d"],
                         "d2h_bytes_per_step": 32},
                 "step_tflops": fo["step"] * mo["B"] / (mo["ms_step"] / 1e3) / 1e12, "gpu_launches_per_step": mo["launches"],

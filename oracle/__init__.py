@@ -17,7 +17,7 @@ Pinning: the reference ships no tests, golden vectors or fixtures for this path 
 8c), so parity is pinned against the reference ITSELF run in the build container: make_golden.py imports
 the unmodified reference nn.Modules from /root/reference (through ref_shim.py, which only stubs the
 absent basicsr/kornia imports) and writes tests/golden/*.pt; tests/test_oracle.py checks nets.py against
-those files (and against the live reference when /root/reference is present).  The basicsr-side pieces
+those files (make_golden_ref.py records the remaining reference results the tests compare with).  The basicsr-side pieces
 (losses, USM, Adam/EMA wiring) have no runnable reference here: they are "parity unpinned" by the
 reference and are cross-checked against the torch / torchvision / cv2 primitives they wrap.
 """

@@ -5,6 +5,7 @@ shard reader and compares with these digests, so the parity claim travels to mac
 
 python oracle/make_golden_data.py   # -> tests/golden/data_synthetic_tree.json
 """
+import glob
 import hashlib
 import importlib
 import json
@@ -34,13 +35,14 @@ def main():
     sys.path.insert(0, REF)
     ref_cls = importlib.import_module("ssr.data.s2-naip_dataset").S2NAIPDataset
     import test_data_cpu as t
+    glob.glob = t.sorted_glob             # the test replays in name order, whatever order this file system lists
     golden = {}
     for variant in t.VARIANTS:
         root = tempfile.mkdtemp(prefix="ssr_golden_")
         t.make_tree(root, with_old=(variant == "old_hr"))
         random.seed(99)
         ds = ref_cls(t.opts(root, **t.variant_options(variant, root)))
-        # the samples depend on the directory listing order (it fixes which random numbers each chip sees): record it
+        # the samples depend on the listing order (it fixes which random numbers each chip sees): record it
         golden[variant] = {"order": [dp[2] for dp in ds.datapoints], "items": [digest(s) for s in t.collect(ds, 1234)]}
     path = os.path.join(ROOT, "tests", "golden", "data_synthetic_tree.json")
     with open(path, "w") as fh:

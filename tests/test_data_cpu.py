@@ -4,22 +4,27 @@ A small synthetic S2-NAIP tree (PNG files, written with cv2) exercises every bra
 black pixel (rejected), Sentinel-2 frames with black pixels (used only to fill up), a chip with too few frames, a missing band
 file, the random-crop augmentation, `train_samples` sub-sampling and `old_naip_path`.  With the same `random` seed
   * the shard reader returns the same tensors as the PNG reader of the same class, and
-  * -- when /root/reference is present -- both return what the UNMODIFIED reference `S2NAIPDataset` returns,
-    item by item, including the indices it skips to.
+  * both return what the UNMODIFIED reference `S2NAIPDataset` returned (tests/golden/data_synthetic_tree.json), item by item,
+    including the indices it skips to.
 """
+import glob
 import os
 import random
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
 cv2 = pytest.importorskip("cv2")
-REF = "/root/reference"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 N_S2 = 4
+_glob = glob.glob
+
+
+def sorted_glob(*args, **kwargs):
+    """glob.glob in name order.  The datasets list chips in glob order, and the order fixes which random numbers each chip
+    draws; directory order differs between file systems, so the fixture is recorded and replayed in name order."""
+    return sorted(_glob(*args, **kwargs))
 
 
 def _write_png(path, chw):
@@ -77,36 +82,6 @@ def assert_same(a, b):
                 assert x[k].dtype == torch.uint8 and x[k].shape == y[k].shape and torch.equal(x[k], y[k]), k
 
 
-REFERENCE_CHECK = r"""
-import importlib, os, random, sys, torch
-sys.path.insert(0, {root!r}); sys.path.insert(0, os.path.join({root!r}, "tests"))
-from satlas_super_resolution_b200 import dropin
-dropin.install()                      # registry / scandir stand-ins for the absent basicsr; seeds sys.modules (hence the subprocess)
-sys.path.insert(0, {ref!r})
-ref_cls = importlib.import_module("ssr.data.s2-naip_dataset").S2NAIPDataset
-import test_data_cpu as t
-from satlas_super_resolution_b200.data import S2NAIPShardDataset
-tree, prefix, extra = {tree!r}, {prefix!r}, {extra!r}
-def build(cls, **kw):
-    random.seed(99)
-    return cls(t.opts(tree, **extra, **kw))
-ref = t.collect(build(ref_cls), 1234)
-ours = t.collect(build(S2NAIPShardDataset, shard_path=prefix), 1234)
-t.assert_same(ref, ours)
-print("REFERENCE-OK", len(ref))
-"""
-
-
-def check_against_reference(tree, prefix, extra):
-    """the unmodified reference S2NAIPDataset on the PNG tree vs our shard reader, same seeds, in a fresh interpreter"""
-    if not os.path.isdir(os.path.join(REF, "ssr", "data")):
-        return False
-    code = REFERENCE_CHECK.format(root=ROOT, ref=REF, tree=tree, prefix=prefix, extra=extra)
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "REFERENCE-OK" in r.stdout, r.stdout[-2000:] + r.stderr[-4000:]
-    return True
-
-
 VARIANTS = ["plain", "rand_crop", "subset", "old_hr"]
 
 
@@ -116,14 +91,12 @@ def variant_options(variant, root):
 
 
 def check_against_golden(variant, samples, order):
-    """digests recorded from the unmodified reference dataset by oracle/make_golden_data.py (travels without /root/reference);
-    only meaningful when this file system lists the chips in the order the fixture was recorded with"""
+    """digests recorded from the unmodified reference dataset by oracle/make_golden_data.py, chips listed in name order"""
     import hashlib
     import json
     with open(os.path.join(ROOT, "tests", "golden", "data_synthetic_tree.json")) as fh:
         gold = json.load(fh)["variants"][variant]
-    if gold["order"] != order:
-        return False
+    assert gold["order"] == order
     want = gold["items"]
     assert len(want) == len(samples)
     for w, s in zip(want, samples):
@@ -133,12 +106,12 @@ def check_against_golden(variant, samples, order):
             if k in w:
                 assert w[k]["shape"] == list(s[k].shape)
                 assert w[k]["sha256"] == hashlib.sha256(s[k].contiguous().numpy().tobytes()).hexdigest(), (variant, s["Chip"], k)
-    return True
 
 
 @pytest.mark.parametrize("variant", VARIANTS)
-def test_shard_reader_matches_png_reader_and_reference(tmp_path, variant):
+def test_shard_reader_matches_png_reader_and_reference(tmp_path, monkeypatch, variant):
     from satlas_super_resolution_b200.data import S2NAIPShardDataset, pack_s2naip
+    monkeypatch.setattr(glob, "glob", sorted_glob)
     root = str(tmp_path)
     make_tree(root, with_old=(variant == "old_hr"))
     extra = variant_options(variant, root)
@@ -157,9 +130,7 @@ def test_shard_reader_matches_png_reader_and_reference(tmp_path, variant):
     assert s0["lr"].shape == (N_S2 * 4, 32, 32) and s0["hr"].shape == (3, 128, 128)
     # the datapoint with the black NAIP pixel is never returned; the one with too few frames neither
     assert all(s["Chip"] not in ("12_22", "14_24") for s in shard)
-    pinned = check_against_golden(variant, shard, [rec["chip"] for rec in shard_ds.datapoints])
-    pinned = check_against_reference(root, prefix, extra) or pinned
-    assert pinned, "neither the golden fixture (directory order differs) nor the live reference could pin this run"
+    check_against_golden(variant, shard, [rec["chip"] for rec in shard_ds.datapoints])
 
 
 def test_frame_choice_prefers_clean_frames(tmp_path):

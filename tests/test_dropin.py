@@ -1,5 +1,5 @@
-"""CPU tests of the drop-in boundary: registry surface, constructor signatures, state_dict key schema, and -- when
-/root/reference is present -- that the reference's own package scanners and builders return OUR classes."""
+"""CPU tests of the drop-in boundary: registry surface, constructor signatures, state_dict key schema, and that the
+reference's package scanners and builders return OUR classes."""
 import os
 import subprocess
 import sys
@@ -8,7 +8,6 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 def test_registry_surface_and_schema():
@@ -54,28 +53,32 @@ def test_unsupported_options_fail_loudly():
         losses.PerceptualLoss({"conv5_4": 1.0}, style_weight=1.0)
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "ssr")), reason="/root/reference only exists in the build container")
 def test_reference_scanners_pick_up_our_classes():
-    """run in a subprocess: dropin.install() then import the reference's `ssr` package exactly as ssr/infer.py does"""
+    """run in a subprocess: dropin.install(), then what the reference's arch scanner (ssr/archs/__init__.py) and
+    ssr/utils/model_utils.build_network do with ssr/options/infer_example.yml.  The scanned module names, the options and the
+    reference generator's state_dict keys were recorded from the reference (oracle/make_golden_ref.py)."""
     code = r'''
-import sys
+import importlib, json, sys
 sys.path.insert(0, %r)
 import satlas_super_resolution_b200.dropin as dropin
-dropin.install(reference_root=%r)
-import ssr.archs                                   # the reference's scanner (ssr/archs/__init__.py)
-from ssr.utils.model_utils import build_network    # what ssr/infer.py:11 imports
-from ssr.utils.infer_utils import format_s2naip_data, stitch
-from ssr.utils.options import yaml_load
+dropin.install()
 from basicsr.utils.registry import ARCH_REGISTRY
 from satlas_super_resolution_b200 import archs
+with open(%r) as fh:
+    gold = json.load(fh)
+assert {"rrdbnet_arch", "discriminator_arch"} <= set(gold["arch_modules"])
+mods = {n: importlib.import_module(f"ssr.archs.{n}") for n in ("rrdbnet_arch", "discriminator_arch")}   # as the scanner imports them
+assert mods["rrdbnet_arch"].SSR_RRDBNet is archs.SSR_RRDBNet, "the scanner does not import the engine module"
+assert mods["discriminator_arch"].SSR_UNetDiscriminatorSN is archs.SSR_UNetDiscriminatorSN
 assert ARCH_REGISTRY.get("SSR_RRDBNet") is archs.SSR_RRDBNet, "registry does not hold the engine class"
 assert ARCH_REGISTRY.get("SSR_UNetDiscriminatorSN") is archs.SSR_UNetDiscriminatorSN
-opt = yaml_load(%r)
-m = build_network(opt)
+opt, net = gold["opt"], gold["opt"]["network_g"]
+m = mods["rrdbnet_arch"].SSR_RRDBNet(num_in_ch=int(opt["n_lr_images"]) * 3, num_out_ch=3, num_feat=int(net["num_feat"]),
+                                     num_block=int(net["num_block"]), num_grow_ch=int(net["num_grow_ch"]), scale=int(opt["scale"]))
 assert type(m) is archs.SSR_RRDBNet and m.num_in_ch == int(opt["n_lr_images"]) * 3
-assert "SSR_OSMObjDiscriminator" in ARCH_REGISTRY.keys() or len(list(ARCH_REGISTRY.keys())) >= 3   # the reference's other archs still register
+assert list(m.state_dict().keys()) == gold["state_dict_keys"], "checkpoints of the reference generator would not load"
 print("OK", len(m.state_dict()))
-''' % (ROOT, REF, os.path.join(REF, "ssr/options/infer_example.yml"))
+''' % (ROOT, os.path.join(ROOT, "tests", "golden", "dropin_infer_example.json"))
     res = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert res.returncode == 0, res.stdout + res.stderr
     assert "OK 702" in res.stdout

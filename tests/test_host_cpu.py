@@ -94,13 +94,19 @@ def test_bench_helpers():
     assert "side lane" not in bench.train_rooflines(dict(m, side_lane=False, graph_us={}), 3, 1452.2, "measured")[0]["timing"]
 
 
+def format_s2naip_input():
+    import numpy as np
+    rng = np.random.RandomState(0)
+    s2 = rng.randint(1, 255, size=(10 * 32, 32, 3)).astype(np.uint8)
+    s2[3 * 32 + 5, 7] = 0                       # frame 3 has a pure-black pixel -> "bad"
+    return s2
+
+
 def test_infer_format_matches_reference_semantics():
     import random
     import numpy as np
     from satlas_super_resolution_b200.infer import format_s2naip_data
-    rng = np.random.RandomState(0)
-    s2 = rng.randint(1, 255, size=(10 * 32, 32, 3)).astype(np.uint8)
-    s2[3 * 32 + 5, 7] = 0                       # frame 3 has a pure-black pixel -> "bad"
+    s2 = format_s2naip_input()
     t, first = format_s2naip_data(s2, 8, rng=random.Random(1))
     assert t.shape == (1, 24, 32, 32) and t.dtype == torch.float32 and float(t.max()) <= 1
     assert np.array_equal(first, s2[:32])
@@ -108,19 +114,10 @@ def test_infer_format_matches_reference_semantics():
     frames = {tuple(s2[i * 32:(i + 1) * 32].transpose(2, 0, 1).flatten()[:8]) for i in range(10) if i != 3}
     for k in range(8):
         assert tuple((t[0, 3 * k:3 * k + 3] * 255).round().byte().numpy().flatten()[:8]) in frames
-    ref_path = "/root/reference/ssr/utils/infer_utils.py"
-    if os.path.exists(ref_path):
-        # the live reference function (needs only numpy / torch; skimage import stubbed) with the same seeded global RNG
-        import importlib.util, types
-        sys.modules.setdefault("skimage", types.ModuleType("skimage"))
-        sys.modules.setdefault("skimage.io", types.ModuleType("skimage.io"))
-        spec = importlib.util.spec_from_file_location("_ref_infer_utils", ref_path)
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        random.seed(5)
-        want, want_first = mod.format_s2naip_data(s2, 8, "cpu")
-        got, got_first = format_s2naip_data(s2, 8, rng=random.Random(5))
-        assert torch.equal(want, got) and np.array_equal(want_first, got_first)
+    # what the reference's format_s2naip_data returned for this input after random.seed(5) (oracle/make_golden_ref.py)
+    gold = torch.load(os.path.join(ROOT, "tests", "golden", "format_s2naip_data.pt"))
+    got, got_first = format_s2naip_data(s2, gold["n_s2_images"], rng=random.Random(gold["random_seed"]))
+    assert torch.equal(gold["s2_tensor_u8"].float() / 255, got) and np.array_equal(gold["s2_image"].numpy(), got_first)
 
 
 GLOO_WORKER = r'''

@@ -1,7 +1,7 @@
 """CPU tests: the oracle (oracle/nets.py, oracle/losses.py) is pinned against
-  (1) the golden fixtures produced by the UNMODIFIED reference modules (oracle/make_golden.py, tests/golden/*.pt),
-  (2) the live reference when /root/reference is present (build container only),
-  (3) the torch / torchvision / cv2 primitives the restated basicsr pieces wrap.
+  (1) the golden fixtures produced by the UNMODIFIED reference modules (oracle/make_golden.py, oracle/make_golden_ref.py,
+      tests/golden/*.pt),
+  (2) the torch / torchvision / cv2 primitives the restated basicsr pieces wrap.
 """
 import os
 
@@ -11,7 +11,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from oracle import losses, nets, ref_shim
+from oracle import losses, nets
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -77,27 +77,22 @@ def test_pixel_unshuffle_golden():
     assert torch.equal(nets.pixel_unshuffle(g["x"], 2), F.pixel_unshuffle(g["x"], 2))
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference only exists in the build container")
 def test_oracle_against_live_reference():
-    RRDB, UNetD = ref_shim.reference_archs()
-    sd = nets.rrdbnet_init(24, 3, num_block=1, seed=5)
-    m = RRDB(num_in_ch=24, num_out_ch=3, num_block=1)
-    m.load_state_dict(sd, strict=True)
-    x = torch.rand(1, 24, 32, 32, generator=torch.Generator().manual_seed(6))
+    """against what the reference's SSR_RRDBNet / SSR_UNetDiscriminatorSN produced (oracle/make_golden_ref.py, tests/golden/ref_modules.pt)"""
+    g = load("ref_modules.pt")
+    sd = nets.rrdbnet_init(24, 3, num_block=1, seed=g["sd_seed"])
+    assert [(k, list(v.shape)) for k, v in sd.items()] == g["g1_shapes"]       # what load_state_dict(strict=True) requires
+    x = torch.rand(1, 24, 32, 32, generator=torch.Generator().manual_seed(g["x_seed"]))
     with torch.no_grad():
-        assert torch.allclose(m.eval()(x), nets.rrdbnet_forward(sd, x, num_block=1), atol=1e-5)
+        assert torch.allclose(g["y"], nets.rrdbnet_forward(sd, x, num_block=1), atol=1e-5)
     # the reference's own default init has the distribution oracle.nets restates
-    ref_sd = RRDB(num_in_ch=24, num_out_ch=3, num_block=2).state_dict()
     mine = nets.rrdbnet_init(24, 3, num_block=2, seed=0)
-    assert list(ref_sd.keys()) == list(mine.keys())
-    for k in ("body.0.rdb1.conv1.weight", "conv_first.weight", "body.1.rdb3.conv5.weight"):
-        assert ref_sd[k].shape == mine[k].shape
-        assert abs(ref_sd[k].std().item() / mine[k].std().item() - 1) < 0.1, k
-    assert ref_sd["body.0.rdb2.conv3.bias"].abs().max() == 0
+    assert [(k, list(v.shape)) for k, v in mine.items()] == g["g2_shapes"]
+    for k, std in g["g2_std"].items():
+        assert abs(std / mine[k].std().item() - 1) < 0.1, k
+    assert g["g2_bias_abs_max"] == 0
     dsd = nets.unet_disc_init(27, seed=7)
-    d = UNetD(num_in_ch=27)
-    d.load_state_dict(dsd, strict=True)
-    assert list(d.state_dict().keys()) == list(dsd.keys())
+    assert [(k, list(v.shape)) for k, v in dsd.items()] == g["d_shapes"]
 
 
 # --------------------------------------------------------------------------- restated basicsr pieces vs primitives
