@@ -375,6 +375,22 @@ int ssr_u8_shift_diff_sums(const void* a_u8, const void* b_u8, int32_t b, int32_
  * zeroes out and divides); window11_device = cv2.getGaussianKernel(11, 1.5) as 11 doubles in device memory */
 int ssr_u8_ssim_sums(const void* a_u8, const void* b_u8, int32_t b, int32_t h, int32_t w, int32_t c, int32_t crop_border,
                      const double* window11_device, double* out, void* stream);
+/* LPIPS, lpips 0.1 net='vgg' (calculate_lpips of ssr/metrics/lpips.py:7-21, called from ssr_esrgan_model.py:305-312).
+ * Ingest: uint8 HWC batch [b, h, w, c] -> NHWC bf16 images image_offset .. image_offset + b - 1 of dst (pixel stride dst_pix_stride,
+ * channels [c, c_pad) zero): v = (x / 255 - shift[ch]) / scale[ch] (device floats; lpips' ScalingLayer on x / 255). */
+int ssr_ingest_u8_nhwc(const void* src_u8, int32_t b, int32_t h, int32_t w, int32_t c, void* dst_bf16, int32_t dst_pix_stride,
+                       int32_t image_offset, int32_t c_pad, const float* shift, const float* scale, void* stream);
+/* partial-sum slots per image of one tap of size h x w (a function of h * w only) */
+int32_t ssr_lpips_cta_count(int32_t h, int32_t w);
+/* One tap of the head: feat = [2b, h, w, c] bf16 post-ReLU features (c = 64 / 128 / 256 / 512), pair n = images (n, b + n);
+ * lin_w = lin{k}.model.1.weight as c f32 (device).  partial[n * ssr_lpips_cta_count(h, w) + t] = sum over the pixels of slot t of
+ * sum_ch lin_w[ch] * (f0 / (|f0| + 1e-10) - f1 / (|f1| + 1e-10))^2 (|f| the channel L2 norm).  Fixed summation order, no atomics. */
+int ssr_lpips_layer_sums(const void* feat_bf16, int32_t b, int32_t h, int32_t w, int32_t c, const float* lin_w, double* partial,
+                         void* stream);
+/* out[n] = sum_k (sum of tap k's partials of pair n) / (tap_h[k] * tap_w[k]) in f64, fixed order; the partials of the n_taps (<= 8)
+ * taps lie back to back ([b][cta_count] each); tap_h / tap_w are host arrays */
+int ssr_lpips_finish(const double* partial, int32_t b, int32_t n_taps, const int32_t* tap_h, const int32_t* tap_w, double* out,
+                     void* stream);
 
 #ifdef __cplusplus
 }

@@ -53,6 +53,10 @@ PROTOS = {
     "ssr_f32_nchw_to_u8_hwc": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp]),
     "ssr_u8_shift_diff_sums": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp]),
     "ssr_u8_ssim_sums": (C.c_int, [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp]),
+    "ssr_ingest_u8_nhwc": (C.c_int, [vp, i32, i32, i32, i32, vp, i32, i32, i32, vp, vp, vp]),
+    "ssr_lpips_cta_count": (C.c_int32, [i32, i32]),
+    "ssr_lpips_layer_sums": (C.c_int, [vp, i32, i32, i32, i32, vp, vp, vp]),
+    "ssr_lpips_finish": (C.c_int, [vp, i32, i32, C.POINTER(i32), C.POINTER(i32), vp, vp]),
     "ssr_spectral_norm": (C.c_int, [vp, i32, i32, f32, vp]),
     "ssr_spectral_norm_bwd": (C.c_int, [vp, i32, vp]),
     "ssr_usm_sharp": (C.c_int, [vp, vp, vp, i32, i32, i32, vp, i32, f32, f32, vp]),

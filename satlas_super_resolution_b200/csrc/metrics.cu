@@ -120,6 +120,130 @@ __global__ void u8_ssim_kernel(const uint8_t* __restrict__ a, const uint8_t* __r
   }
 }
 
+// ------------------------------------------------------------------ LPIPS (lpips 0.1, net='vgg'; ssr/metrics/lpips.py:7-21)
+// uint8 HWC image -> the 16-channel NHWC bf16 buffer conv1_1 reads: v = (x / 255 - shift[c]) / scale[c] (lpips ScalingLayer on the
+// [0, 1] values calculate_lpips passes), channels [c, c_pad) zero.  One thread per pixel.
+__global__ void ingest_u8_nhwc_kernel(const uint8_t* __restrict__ src, __nv_bfloat16* __restrict__ dst, long npix, int C, int dst_stride,
+                                      int c_pad, const float* __restrict__ shift, const float* __restrict__ scale) {
+  for (long p = blockIdx.x * (long)blockDim.x + threadIdx.x; p < npix; p += (long)gridDim.x * blockDim.x) {
+    __nv_bfloat16* d = dst + p * dst_stride;
+    for (int g = 0; g < c_pad; g += 8) {
+      __align__(16) __nv_bfloat16 v[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const int c = g + j;
+        float f = 0.f;
+        if (c < C) f = ((float)src[p * C + c] / 255.f - shift[c]) / scale[c];
+        v[j] = __float2bfloat16(f);
+      }
+      *reinterpret_cast<uint4*>(d + g) = *reinterpret_cast<const uint4*>(v);
+    }
+  }
+}
+
+__device__ __forceinline__ void bf16x8_to_f32(const uint4& v, float* f) {
+  const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&v);
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 t = __bfloat1622float2(h[j]);
+    f[2 * j] = t.x;
+    f[2 * j + 1] = t.y;
+  }
+}
+
+constexpr int LPIPS_THREADS = 256;
+constexpr int LPIPS_PIX_PER_CTA = 256;   // the partial-sum slots of an image depend on (h, w) only: batch-invariant by construction
+
+// One tap of the LPIPS head.  x = [2b, h, w, C] post-ReLU features (images n and b + n are the pair); per pixel
+//   d = sum_c lin[c] * (f0[c] / (|f0| + 1e-10) - f1[c] / (|f1| + 1e-10))^2
+// with |f| = sqrt(sum_c f^2).  A group of LPP = min(32, C / 8) lanes owns one pixel, each lane VPL 16-byte vectors of both images held
+// in registers; the two norms and d are butterfly sums over the group (every lane ends with the same bits).  CTA (t, n) covers pixels
+// [t * 256, (t + 1) * 256) of pair n and writes their sum (fixed order, f64) to partial[n * gridDim.x + t].  No atomics.
+template <int C>
+__global__ void __launch_bounds__(LPIPS_THREADS) lpips_layer_sums_kernel(const __nv_bfloat16* __restrict__ x, int B, int hw,
+                                                                         const float* __restrict__ lin, double* __restrict__ partial) {
+  constexpr int LPP = C / 8 < 32 ? C / 8 : 32;
+  constexpr int VPL = C / (8 * LPP);
+  constexpr int GROUPS = LPIPS_THREADS / LPP;
+  const int n = blockIdx.y;
+  const int lane_g = threadIdx.x % LPP, grp = threadIdx.x / LPP;
+  float w[VPL * 8];
+#pragma unroll
+  for (int v = 0; v < VPL; ++v) {
+    const float4 a = *reinterpret_cast<const float4*>(lin + (v * LPP + lane_g) * 8);
+    const float4 b = *reinterpret_cast<const float4*>(lin + (v * LPP + lane_g) * 8 + 4);
+    w[v * 8 + 0] = a.x; w[v * 8 + 1] = a.y; w[v * 8 + 2] = a.z; w[v * 8 + 3] = a.w;
+    w[v * 8 + 4] = b.x; w[v * 8 + 5] = b.y; w[v * 8 + 6] = b.z; w[v * 8 + 7] = b.w;
+  }
+  const __nv_bfloat16* x0 = x + (long)n * hw * C;
+  const __nv_bfloat16* x1 = x + (long)(B + n) * hw * C;
+  const int p_end = min(hw, (blockIdx.x + 1) * LPIPS_PIX_PER_CTA);
+  float acc = 0.f;
+  // the trip count is uniform over the CTA (the shuffles need whole warps); a group past the end reads zeros, which add 0
+  for (int p0 = blockIdx.x * LPIPS_PIX_PER_CTA; p0 < p_end; p0 += GROUPS) {
+    const int p = p0 + grp;
+    float f0[VPL * 8], f1[VPL * 8];
+#pragma unroll
+    for (int v = 0; v < VPL; ++v) {
+      const long off = (long)p * C + (v * LPP + lane_g) * 8;
+      const uint4 z = make_uint4(0u, 0u, 0u, 0u);
+      bf16x8_to_f32(p < p_end ? *reinterpret_cast<const uint4*>(x0 + off) : z, f0 + v * 8);
+      bf16x8_to_f32(p < p_end ? *reinterpret_cast<const uint4*>(x1 + off) : z, f1 + v * 8);
+    }
+    float s0 = 0.f, s1 = 0.f;
+#pragma unroll
+    for (int j = 0; j < VPL * 8; ++j) {
+      s0 = fmaf(f0[j], f0[j], s0);
+      s1 = fmaf(f1[j], f1[j], s1);
+    }
+#pragma unroll
+    for (int off = LPP / 2; off; off >>= 1) {
+      s0 += __shfl_xor_sync(0xffffffffu, s0, off);
+      s1 += __shfl_xor_sync(0xffffffffu, s1, off);
+    }
+    const float r0 = sqrtf(s0) + 1e-10f, r1 = sqrtf(s1) + 1e-10f;
+    float d = 0.f;
+#pragma unroll
+    for (int j = 0; j < VPL * 8; ++j) {
+      const float e = f0[j] / r0 - f1[j] / r1;
+      d = fmaf(w[j], e * e, d);
+    }
+#pragma unroll
+    for (int off = LPP / 2; off; off >>= 1) d += __shfl_xor_sync(0xffffffffu, d, off);
+    acc += d;
+  }
+  // the group's pixel sum -> shared memory, then one thread adds the groups in index order
+  __shared__ double grp_sum[GROUPS];
+  if (lane_g == 0) grp_sum[grp] = (double)acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int g = 0; g < GROUPS; ++g) s += grp_sum[g];
+    partial[(long)n * gridDim.x + blockIdx.x] = s;
+  }
+}
+
+struct LpipsTaps {
+  int n_taps;
+  int ctas[8];
+  int hw[8];
+  long offset[8];   // first partial of tap k (partials of tap k: [b][ctas[k]])
+};
+
+// out[n] = sum_k (sum_t partial_k[n][t]) / hw_k, every sum in f64 in index order
+__global__ void lpips_finish_kernel(const double* __restrict__ partial, int B, LpipsTaps taps, double* __restrict__ out) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= B) return;
+  double total = 0.0;
+  for (int k = 0; k < taps.n_taps; ++k) {
+    const double* p = partial + taps.offset[k] + (long)n * taps.ctas[k];
+    double s = 0.0;
+    for (int t = 0; t < taps.ctas[k]; ++t) s += p[t];
+    total += s / (double)taps.hw[k];
+  }
+  out[n] = total;
+}
+
 }  // namespace ssr
 
 using namespace ssr;
@@ -156,4 +280,58 @@ extern "C" int ssr_u8_ssim_sums(const void* a_u8, const void* b_u8, int32_t b, i
                                                                     b, h, w, c, crop_border, window11_device, out);
   count_launch();
   return check_last("u8_ssim launch") ? SSR_OK : SSR_E_CUDA;
+}
+
+extern "C" int ssr_ingest_u8_nhwc(const void* src_u8, int32_t b, int32_t h, int32_t w, int32_t c, void* dst_bf16, int32_t dst_pix_stride,
+                                  int32_t image_offset, int32_t c_pad, const float* shift, const float* scale, void* stream) {
+  SSR_REQUIRE(src_u8 && dst_bf16 && shift && scale && b > 0 && h > 0 && w > 0 && c > 0 && image_offset >= 0, "ssr_ingest_u8_nhwc: bad args");
+  SSR_REQUIRE(c_pad % 8 == 0 && c_pad >= c && dst_pix_stride % 8 == 0 && dst_pix_stride >= c_pad, "ssr_ingest_u8_nhwc: c_pad/stride");
+  SSR_REQUIRE((reinterpret_cast<uintptr_t>(dst_bf16) & 15) == 0, "ssr_ingest_u8_nhwc: dst alignment");
+  const long npix = (long)b * h * w;
+  __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(dst_bf16) + (long)image_offset * h * w * dst_pix_stride;
+  ingest_u8_nhwc_kernel<<<grid_for_m(npix, 256), 256, 0, STREAM(stream)>>>(reinterpret_cast<const uint8_t*>(src_u8), dst, npix, c, dst_pix_stride,
+                                                                          c_pad, shift, scale);
+  count_launch();
+  return check_last("ingest_u8_nhwc launch") ? SSR_OK : SSR_E_CUDA;
+}
+
+extern "C" int32_t ssr_lpips_cta_count(int32_t h, int32_t w) {
+  return (int32_t)((h * w + LPIPS_PIX_PER_CTA - 1) / LPIPS_PIX_PER_CTA);
+}
+
+extern "C" int ssr_lpips_layer_sums(const void* feat_bf16, int32_t b, int32_t h, int32_t w, int32_t c, const float* lin_w, double* partial,
+                                    void* stream) {
+  SSR_REQUIRE(feat_bf16 && lin_w && partial && b > 0 && h > 0 && w > 0, "ssr_lpips_layer_sums: bad args");
+  SSR_REQUIRE((reinterpret_cast<uintptr_t>(feat_bf16) & 15) == 0 && (reinterpret_cast<uintptr_t>(lin_w) & 15) == 0,
+              "ssr_lpips_layer_sums: alignment");
+  SSR_REQUIRE(b <= 65535, "ssr_lpips_layer_sums: at most 65535 pairs");
+  const dim3 grid((unsigned)ssr_lpips_cta_count(h, w), (unsigned)b);
+  const __nv_bfloat16* x = reinterpret_cast<const __nv_bfloat16*>(feat_bf16);
+  switch (c) {
+    case 64: lpips_layer_sums_kernel<64><<<grid, LPIPS_THREADS, 0, STREAM(stream)>>>(x, b, h * w, lin_w, partial); break;
+    case 128: lpips_layer_sums_kernel<128><<<grid, LPIPS_THREADS, 0, STREAM(stream)>>>(x, b, h * w, lin_w, partial); break;
+    case 256: lpips_layer_sums_kernel<256><<<grid, LPIPS_THREADS, 0, STREAM(stream)>>>(x, b, h * w, lin_w, partial); break;
+    case 512: lpips_layer_sums_kernel<512><<<grid, LPIPS_THREADS, 0, STREAM(stream)>>>(x, b, h * w, lin_w, partial); break;
+    default: SSR_REQUIRE(false, "ssr_lpips_layer_sums: c must be 64, 128, 256 or 512 (got %d)", c);
+  }
+  count_launch();
+  return check_last("lpips_layer_sums launch") ? SSR_OK : SSR_E_CUDA;
+}
+
+extern "C" int ssr_lpips_finish(const double* partial, int32_t b, int32_t n_taps, const int32_t* tap_h, const int32_t* tap_w, double* out,
+                                void* stream) {
+  SSR_REQUIRE(partial && out && tap_h && tap_w && b > 0 && n_taps > 0 && n_taps <= 8, "ssr_lpips_finish: bad args (1..8 taps)");
+  LpipsTaps t;
+  t.n_taps = n_taps;
+  long off = 0;
+  for (int k = 0; k < n_taps; ++k) {
+    SSR_REQUIRE(tap_h[k] > 0 && tap_w[k] > 0, "ssr_lpips_finish: bad tap size");
+    t.ctas[k] = ssr_lpips_cta_count(tap_h[k], tap_w[k]);
+    t.hw[k] = tap_h[k] * tap_w[k];
+    t.offset[k] = off;
+    off += (long)b * t.ctas[k];
+  }
+  lpips_finish_kernel<<<(b + 127) / 128, 128, 0, STREAM(stream)>>>(partial, b, t, out);
+  count_launch();
+  return check_last("lpips_finish launch") ? SSR_OK : SSR_E_CUDA;
 }

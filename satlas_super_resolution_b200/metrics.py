@@ -1,5 +1,5 @@
-"""Batched validation metrics on the GPU: PSNR, SSIM (basicsr.metrics.psnr_ssim) and cPSNR (ssr/metrics/cpsnr.py:7-59) for a whole
-batch of (SR, ground truth) pairs at once -- the reference's nondist_validation (ssr/models/ssr_esrgan_model.py:296-345) converts
+"""Batched validation metrics on the GPU: PSNR, SSIM (basicsr.metrics.psnr_ssim), cPSNR (ssr/metrics/cpsnr.py:7-59) and LPIPS-VGG
+(ssr/metrics/lpips.py:7-21, through lpips.LPIPSEngine) for a whole batch of (SR, ground truth) pairs at once -- the reference's nondist_validation (ssr/models/ssr_esrgan_model.py:296-345) converts
 one image at a time with tensor2img and runs numpy on the host (cPSNR: an 81-offset brute-force search per image).
 
 PSNR / cPSNR: the device returns EXACT integer sums of the uint8 differences (ssr_u8_shift_diff_sums); the float64 formulas of the
@@ -87,7 +87,50 @@ def calculate_ssim(img, img2, crop_border, input_order="HWC", test_y_channel=Fal
     return (out / n).mean(dim=1).cpu().tolist()
 
 
-for _f in (calculate_psnr, calculate_ssim, calculate_cpsnr):
+def check_lpips_model(lpips_model):
+    """only lpips_model 'vgg' is built (AlexNet's 11 x 11 stride-4 / 5 x 5 convs are shapes no kernel of the engine takes)"""
+    if lpips_model != "vgg":
+        raise NotImplementedError(f"calculate_lpips: lpips_model={lpips_model!r} is not built (only lpips_model: vgg runs on the GPU "
+                                  "engine; 'alexnet' and a missing lpips_model are not supported)")
+
+
+_LPIPS_ENGINES = {}      # (device, weight source) -> lpips.LPIPSEngine
+
+
+def lpips_engine(device, lpips_seed=None):
+    """the LPIPS engine of `device` for the weights lpips_weight_source() finds, built once and reused"""
+    from . import weights
+    from .lpips import LPIPSEngine
+    device = torch.device(device)
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    source = weights.lpips_weight_source(lpips_seed)
+    key = (str(device), source)
+    eng = _LPIPS_ENGINES.get(key)
+    if eng is None:
+        vgg, lin = weights.load_lpips_state(source)
+        eng = _LPIPS_ENGINES[key] = LPIPSEngine(vgg, lin, device)
+    return eng
+
+
+def calculate_lpips(img, img2, lpips_model=None, lpips_seed=None, **kwargs):
+    """ssr/metrics/lpips.py calculate_lpips over a batch -> list of floats: lpips.LPIPS(net='vgg') of img[i] / 255 against img2[i] / 255
+    (uint8 [B, H, W, 3] cuda batches from to_uint8_images; BGR order and [0, 1] range as the reference passes them).
+    lpips_seed: seeded random weights when the pretrained files are absent (tests / benchmarks)."""
+    check_lpips_model(lpips_model)
+    from .lpips import check_size
+    assert img.shape == img2.shape, f"Image shapes are different: {tuple(img.shape)}, {tuple(img2.shape)}."
+    check_size(img.shape[1], img.shape[2])
+    return lpips_engine(img.device, lpips_seed).distance(img, img2)
+
+
+def check_metric_opt(opt):
+    """option checks that can fail before any image is processed"""
+    if opt.get("type") == "calculate_lpips":
+        check_lpips_model(opt.get("lpips_model"))
+
+
+for _f in (calculate_psnr, calculate_ssim, calculate_cpsnr, calculate_lpips):
     _register(METRIC_REGISTRY, _f)
 
 

@@ -239,7 +239,8 @@ class SSRESRGANModel:
 
     def nondist_validation(self, dataloader, current_iter, tb_logger, save_img):
         """The loop of ssr_esrgan_model.py:269-352 with the per-image host work batched on the GPU: EMA-generator forward
-        (test()), tensor2img, and PSNR / SSIM / cPSNR for the whole validation batch at once (metrics.py).  Any batch size works
+        (test()), tensor2img, and PSNR / SSIM / cPSNR / LPIPS for the whole validation batch at once (metrics.py); metric options are
+        checked before the first batch.  Any batch size works
         (the reference's loop assumes 1); results are averaged over images.  Image dumps (`save_img`) are PNG IO outside the hot
         path and are not written."""
         from . import metrics as M
@@ -252,8 +253,9 @@ class SSRESRGANModel:
             for name, mopt in metrics2run.items():
                 if mopt["type"] not in M.METRIC_REGISTRY:
                     raise NotImplementedError(f"metric '{mopt['type']}' ({name}) is outside the built path (calculate_psnr / "
-                                              "calculate_ssim / calculate_cpsnr run batched on the GPU; LPIPS / CLIPScore need "
-                                              "pretrained networks that are not part of this engine)")
+                                              "calculate_ssim / calculate_cpsnr / calculate_lpips run batched on the GPU; "
+                                              "CLIPScore needs CLIP ViT checkpoints that are not part of this engine)")
+                M.check_metric_opt(mopt)
             self.metric_results = {metric: 0.0 for metric in metrics2run}
             self._initialize_best_metric_results(dataset_name, metrics2run)
         n_img = 0
